@@ -2,7 +2,7 @@
 """bench.py -- ESKF frames/s and residuals/s of the FAST-LIVO measurement + iterated-ESKF hot
 path on B200 (BASELINE.json metric), with the reference-equivalent CPU path timed beside it.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C2] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload C2] [--impl reference] [--dump-outputs DIR]
 
 A *step* is one frame: one full LIO update (all passes, kNN on the rematch passes) followed by
 one full VIO update (ComputeJ: 3 pyramid levels) whose prior is the LIO posterior, on one
@@ -169,16 +169,31 @@ def cpu_frame_runner(po, frame, nthreads, tree="build"):
     lprm = po.lio_params(frame, pc["lio_T"], nthreads=nthreads, early_stop=False)
     vprm = po.vio_params(frame, pc["vio_T"], early_stop=False, force_all_passes=True) if vio else None
 
-    def run():
+    def run(reports=None):
         x = po.state_from_frame(frame)
         lrep = lio.update(lprm, x, x.copy())
+        vrep = None
         rows = lrep.rows_total
         if vio:
             vrep = vio.update(vprm, x, x.copy())
             rows += vrep.rows_total
+        if reports is not None:
+            reports[:] = [lrep, vrep]
         return x, rows
     kind = "reference kNN (ikd_Tree.cpp via oracle/_ref) + line-cited C++ port of the rest" if tree else "port (brute-force kNN)"
     return run, kind
+
+
+def dump_outputs(out_dir, x, lrep, vrep):
+    """--dump-outputs: what the last timed step returned to its caller, one float64 .npy per array: the state (rotation,
+    position, velocity, gyro / accelerometer biases, gravity), its 18x18 covariance and the two update reports."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"state": x.vector(), "cov": x.P,
+              "lio_report": [lrep.passes, lrep.knn_passes, lrep.n_eff_last, lrep.res_mean_last, lrep.rows_total, lrep.converged_last]}
+    if vrep is not None:
+        arrays["vio_report"] = [*vrep.passes, *vrep.last_error, vrep.rows_total, vrep.skipped_last, vrep.cov_updated]
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float64))
 
 
 def cpu_one_frame_child(name):
@@ -288,10 +303,13 @@ def run_reference(args):
         run()
     t0 = time.perf_counter()
     rows = 0
+    reports = []
     for _ in range(args.steps):
-        _, r = run()
+        x, r = run(reports)
         rows += r
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, x, *reports)
     fps = args.steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": fps, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -653,7 +671,8 @@ def measure_full_frame(flb, torch, name, local, dev, stream, flush, steps=20, ra
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=1000)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 1000; 30 with --impl reference, whose CPU "
+                                                                "frames take 0.1-1 s each)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--workload", default="C2", choices=["C1", "C2", "C3", "C4", "T0", "T1"])
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
@@ -664,14 +683,19 @@ def main():
     ap.add_argument("--quick", action="store_true", help="profiling aid: skip the e2e / profile / cpu_baseline legs")
     ap.add_argument("--no-others", action="store_true", help="skip the other_workloads (C3, C4) and batched legs")
     ap.add_argument("--cell-size", type=float, default=0.0, help="experiment: kNN grid cell size (default 2 x the map pitch)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the state, covariance and reports of the last timed step to DIR/<name>.npy (float64), so "
+                         "that two builds can be compared output for output (the inputs are seeded)")
     ap.add_argument("--cpu-one-frame", default=None, help=argparse.SUPPRESS)      # child process of measure_other_workload
     ap.add_argument("--cpu-baseline-child", default=None, help=argparse.SUPPRESS)  # child process of the cpu_baseline leg
     args = ap.parse_args()
+    if args.steps is None:
+        args.steps = 30 if args.impl == "reference" else 1000
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
-        if args.steps > 30:
-            args.steps = 30           # bounded sample: the CPU arm needs ~0.1-1 s per frame
         return run_reference(args)
 
     if args.cpu_one_frame:
@@ -730,6 +754,9 @@ def main():
     total_ms, launches, t_wall = rig.time_resident(args.steps)
     clocks = sampler.stop() if sampler else None
     fps = args.steps / (total_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        xd, ld, vd = h.state_download()          # every rank holds the same state (bit-identical, see parity)
+        dump_outputs(args.dump_outputs, xd, ld, vd if has_vio else None)
 
     trace = rig.pass_trace() if world == 1 else None
     if args.quick:

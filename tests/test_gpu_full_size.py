@@ -1,23 +1,13 @@
 """GPU tier at BASELINE.json's full sizes (C1..C4): the whole frame against the CPU path (oracle +
-the reference's ikd-Tree), plus size-independent properties (sortedness, idempotence, symmetry)."""
+the reference's ikd-Tree, its results pinned in tests/golden/ref_ikdtree.npz by tests/golden/make_golden_ref.py),
+plus size-independent properties (sortedness, idempotence, symmetry)."""
 import numpy as np
 import pytest
 
 from conftest import bits
+from golden_util import digest, load_ref_golden
 
 pytestmark = pytest.mark.gpu
-
-
-def _frame_cpu(po, f, tree):
-    cfg = f["cfg"]
-    lio = po.Lio(f["map_xyz"], f["scan_body"], tree)
-    x = po.state_from_frame(f)
-    lrep = lio.update(po.lio_params(f, cfg.lio_passes - 1, nthreads=8, early_stop=False), x, x.copy())
-    vrep = None
-    if cfg.n_patch:
-        vio = po.Vio(f["image"], f["patch_pos"], f["patch_ref"], f["patch_level"], f["cam"])
-        vrep = vio.update(po.vio_params(f, cfg.vio_passes, early_stop=False, force_all_passes=True), x, x.copy())
-    return x, lrep, vrep
 
 
 def _frame_gpu(flb, h, f):
@@ -31,23 +21,22 @@ def _frame_gpu(flb, h, f):
 
 
 @pytest.mark.parametrize("name", ["C1", "C2", "C3", "C4"])
-def test_full_size_frame_matches_cpu_path(flb, po, name):
-    if po.ref_lib() is None:
-        pytest.skip("needs oracle/_ref/libikdtree_ref.so (brute-force kNN is too slow at this size)")
+def test_full_size_frame_matches_cpu_path(flb, name):
+    gold = load_ref_golden()
+    key = f"frame_{name}"
     f = flb.synth.make_frame(name)
     cfg = f["cfg"]
-    tree = po.IkdTreeRef(f["map_xyz"])
-    xo, lo, vo = _frame_cpu(po, f, tree)
     h = flb.Handle(device=0, cell_size=cfg.cell_size)
     h.load_frame(f)
     xg, lg, vg = _frame_gpu(flb, h, f)
-    assert (lg.passes, lg.knn_passes, lg.n_eff_last, lg.rows_total) == (lo.passes, lo.knn_passes, lo.n_eff_last, lo.rows_total)
-    if vo is not None:
-        assert list(vg.passes) == list(vo.passes) and vg.rows_total == vo.rows_total
-        np.testing.assert_allclose(list(vg.last_error), list(vo.last_error), rtol=1e-6)
-    rel = np.abs(xg.vector() - xo.vector()).max() / np.abs(xo.vector()).max()
+    assert [lg.passes, lg.knn_passes, lg.n_eff_last, lg.rows_total] == list(gold[f"{key}_lio_report"])
+    if vg is not None:
+        assert [*vg.passes, vg.rows_total] == list(gold[f"{key}_vio_report"])
+        np.testing.assert_allclose(list(vg.last_error), gold[f"{key}_vio_last_error"], rtol=1e-6)
+    xo = gold[f"{key}_state"]
+    rel = np.abs(xg.vector() - xo).max() / np.abs(xo).max()
     assert rel < 1e-9, rel                      # bar (north_star): 1e-5
-    np.testing.assert_allclose(xg.P, xo.P, rtol=1e-6, atol=1e-14)
+    np.testing.assert_allclose(xg.P, gold[f"{key}_cov"], rtol=1e-6, atol=1e-14)
     # idempotence: the same update on the same inputs gives the same bits (deterministic reductions)
     xg2, _, _ = _frame_gpu(flb, h, f)
     assert (bits(xg2.vector()) == bits(xg.vector())).all() and (bits(xg2.P) == bits(xg.P)).all()
@@ -74,12 +63,11 @@ def test_full_size_knn_and_pass_properties(flb, po):
     d = (q - nb).astype(np.float32)
     rec = (d[..., 0] * d[..., 0] + d[..., 1] * d[..., 1]) + d[..., 2] * d[..., 2]
     assert (bits(rec) == bits(d2)).all()
-    # exactness against the reference's own ikd-Tree on the full scan
-    if po.ref_lib() is not None:
-        ri, rd = po.IkdTreeRef(f["map_xyz"]).knn(g["world"], nthreads=8)
-        okr = rd[:, 4] <= 5.0
-        assert (okr == ok).all()
-        assert (g["nn_idx"][ok] == ri[ok]).all() and (bits(g["nn_d2"][ok]) == bits(rd[ok])).all()
+    # exactness against the reference's own ikd-Tree on the full scan (world points = the oracle's, bit for bit)
+    gold = load_ref_golden()
+    assert digest(g["world"]) == gold["scanknn_C2_world_digest"]
+    assert ok.sum() == gold["scanknn_C2_n_ok"] and digest(ok) == gold["scanknn_C2_ok_digest"]
+    assert digest(g["nn_idx"][ok].astype(np.int32), g["nn_d2"][ok].astype(np.float32)) == gold["scanknn_C2_digest"]
     # normal equations: symmetric, PSD, and consistent with the exported rows
     H = g["rows"]
     np.testing.assert_allclose(g["HTH"], H.T @ H, rtol=1e-10, atol=1e-9)

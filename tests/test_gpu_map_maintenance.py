@@ -1,78 +1,53 @@
 """GPU tier, SURVEY.md section 8 row f1: device-resident map maintenance against the reference's own ikd-Tree
-(oracle/_ref): Add_Points(downsample = true) (ikd_Tree.cpp:382-457) and Delete_Point_Boxes (:501-521)."""
+(its results pinned in tests/golden/ref_ikdtree.npz by tests/golden/make_golden_ref.py): Add_Points(downsample = true)
+(ikd_Tree.cpp:382-457) and Delete_Point_Boxes (:501-521)."""
 import numpy as np
 import pytest
 
 from conftest import bits
+from golden_util import add_points_case, delete_boxes_case, digest, load_ref_golden, rows_sorted
 
 pytestmark = pytest.mark.gpu
 
 
-def _rows(a):
-    """Sorted view of an (n,3) float32 array as rows, for exact set comparison."""
-    a = np.ascontiguousarray(a, np.float32)
-    v = a.view(np.dtype((np.void, 12))).ravel()
-    return np.sort(v)
-
-
-def _world_scan(f):
-    return ((f["R_true"] @ (f["R_LI"] @ f["scan_body"].T.astype(np.float64) + f["t_LI"][:, None])).T + f["p_true"]).astype(np.float32)
-
-
 @pytest.mark.parametrize("name,ds", [("T0", 0.3), ("T1", 0.3), ("T1", 0.5), ("C2", 0.3)])
-def test_add_points_matches_reference_ikdtree(flb, po, name, ds):
-    if po.ref_lib() is None:
-        pytest.skip("needs oracle/_ref/libikdtree_ref.so")
+def test_add_points_matches_reference_ikdtree(flb, name, ds):
+    gold = load_ref_golden()
+    key = f"add_{name}_{ds}"
     f = flb.synth.make_frame(name)
-    tree = po.IkdTreeRef(f["map_xyz"])
     h = flb.Handle(device=0, cell_size=f["cfg"].cell_size)
     h.map_upload(f["map_xyz"])
-    rng = np.random.default_rng(3)
-    new = _world_scan(f)
-    # three successive batches (the second re-observes the same surfaces, the third is far-field clutter)
-    batches = [new, new + rng.normal(0, 0.02, new.shape).astype(np.float32),
-               rng.uniform(f["map_xyz"].min(0), f["map_xyz"].max(0), (len(new) // 4, 3)).astype(np.float32)]
-    for b in batches:
-        tree.add_points(b, ds)
+    batches, q = add_points_case(f)
+    for b, n_ref, set_ref in zip(batches, gold[f"{key}_counts"], gold[f"{key}_set_digests"]):
         h.map_add_points(b, ds)
-        ref, got = tree.points(), h.map_download()
-        assert len(got) == len(ref)
-        assert (_rows(got) == _rows(ref)).all()
+        got = h.map_download()
+        assert len(got) == n_ref
+        assert digest(rows_sorted(got)) == set_ref
     # the refreshed device grid answers kNN exactly like the refreshed reference tree
-    q = (new[rng.integers(0, len(new), 2000)] + rng.normal(0, 0.1, (2000, 3))).astype(np.float32)
-    ri, rd = tree.knn(q, nthreads=8)
     gi, gd = h.knn(q)
-    ok = rd[:, 4] <= 5.0
-    assert ok.sum() > 1500
-    assert (bits(gd[ok]) == bits(rd[ok])).all()
     m = h.map_download()
-    ref_pts = tree.points()
-    # neighbour identity by coordinates (index spaces differ)
-    # reference returns indices of ITS build order only for original points; compare coordinates instead
+    ok = gd[:, 4] <= 5.0
+    assert ok.sum() == gold[f"{key}_n_ok"] > 1500
+    assert digest(ok) == gold[f"{key}_ok_digest"]
+    assert digest(gd[ok]) == gold[f"{key}_d2_digest"]
+    # neighbour identity by coordinates (index spaces differ): distances recomputed from the returned neighbours
     got_nb = m[gi[ok]]
     d = (q[ok][:, None, :] - got_nb).astype(np.float32)
     rec = (d[..., 0] * d[..., 0] + d[..., 1] * d[..., 1]) + d[..., 2] * d[..., 2]
-    assert (bits(rec) == bits(rd[ok])).all()
-    assert len(ref_pts) == len(m)
+    assert (bits(rec) == bits(gd[ok])).all()
     h.close()
 
 
 def test_delete_boxes_matches_reference_ikdtree(flb, po):
-    if po.ref_lib() is None:
-        pytest.skip("needs oracle/_ref/libikdtree_ref.so")
+    gold = load_ref_golden()
     f = flb.synth.make_frame("T1")
-    tree = po.IkdTreeRef(f["map_xyz"])
     h = flb.Handle(device=0)
     h.map_upload(f["map_xyz"])
-    lo, hi = f["map_xyz"].min(0), f["map_xyz"].max(0)
-    boxes = np.array([[lo[0], lo[1], lo[2], lo[0] + 6, lo[1] + 40, hi[2] + 1],      # a slab along one wall
-                      [0.0, 0.0, -1.0, 4.0, 4.0, 3.0],                              # a chunk in the middle
-                      [hi[0] - 0.01, lo[1], lo[2], hi[0] + 1, hi[1] + 1, hi[2] + 1]], np.float32)
-    n_ref = tree.delete_boxes(boxes)
-    h.map_delete_boxes(boxes)
-    ref, got = tree.points(), h.map_download()
-    assert n_ref > 100 and len(got) == len(ref) == len(f["map_xyz"]) - n_ref
-    assert (_rows(got) == _rows(ref)).all()
+    n_ref = int(gold["delete_T1_n_deleted"])
+    h.map_delete_boxes(delete_boxes_case(f))
+    got = h.map_download()
+    assert n_ref > 100 and len(got) == gold["delete_T1_count"] == len(f["map_xyz"]) - n_ref
+    assert digest(rows_sorted(got)) == gold["delete_T1_set_digest"]
     # LIO still runs on the pruned map and agrees with the oracle on the same point set
     h.scan_upload(f["scan_body"])
     lio = po.Lio(got, f["scan_body"])

@@ -6,6 +6,7 @@ import numpy as np
 import pytest
 
 from conftest import bits
+from golden_util import digest, knn_queries, load_ref_golden, tie_lattice
 
 pytestmark = pytest.mark.gpu
 
@@ -49,16 +50,17 @@ def test_knn_bit_exact(flb, po, frames, handle, name):
 
 
 def test_knn_vs_reference_ikdtree(flb, po, frames, handle):
-    """Same neighbours as the reference's own KD_TREE::Nearest_Search (oracle/_ref)."""
-    if po.ref_lib() is None:
-        pytest.skip("oracle/_ref/libikdtree_ref.so not built")
+    """Same neighbours as the reference's own KD_TREE::Nearest_Search (its results pinned in tests/golden/ref_ikdtree.npz;
+    every query there has 5 neighbours within the 5 m^2 bound)."""
+    gold = load_ref_golden()
     f = frames("T1")
     handle.map_upload(f["map_xyz"])
-    tree = po.IkdTreeRef(f["map_xyz"])
-    rng = np.random.default_rng(17)
-    q = (f["map_xyz"][rng.integers(0, len(f["map_xyz"]), 5000)] + rng.normal(0, 0.3, (5000, 3))).astype(np.float32)
-    ri, rd = tree.knn(q)
+    q = knn_queries(f["map_xyz"], np.random.default_rng(17), 5000, 0.3)
+    ri = gold["knn5000_T1_idx"].astype(np.int32)
     gi, gd = handle.knn(q)
+    d = f["map_xyz"][ri] - q[:, None, :]
+    rd = ((d[..., 0] * d[..., 0] + d[..., 1] * d[..., 1]) + d[..., 2] * d[..., 2]).astype(np.float32)
+    assert digest(rd) == gold["knn5000_T1_d2_digest"]          # the distances the tree returned, recomputed from its indices
     ok = rd[:, 4] <= 5.0
     assert ok.sum() > 4000
     assert (gi[ok] == ri[ok]).all() and (bits(gd[ok]) == bits(rd[ok])).all()
@@ -71,16 +73,10 @@ def test_knn_exact_ties_vs_reference_ikdtree(flb, po, handle):
     the data (ikd_Tree.h:57-60 only orders the heap).  What IS defined, and asserted: the five distances agree bit
     for bit at every rank, every returned index is a true neighbour at exactly that distance, and the two index
     lists differ only inside groups of exactly tied distances."""
-    if po.ref_lib() is None:
-        pytest.skip("oracle/_ref/libikdtree_ref.so not built")
-    g = np.arange(-8, 9, dtype=np.float32) * 0.25
-    lat = np.stack(np.meshgrid(g, g, g[:5], indexing="ij"), -1).reshape(-1, 3).astype(np.float32)
-    rng = np.random.default_rng(3)
-    lat = lat[rng.permutation(len(lat))]
+    lat, q = tie_lattice()
     handle.map_upload(lat)
-    tree = po.IkdTreeRef(lat)
-    q = np.concatenate([lat[:400], lat[400:800] + np.float32(0.125), lat[800:1000] + np.array([0.125, 0, 0], np.float32)]).astype(np.float32)
-    ri, rd = tree.knn(q)
+    gold = load_ref_golden()
+    ri, rd = gold["ties_idx"], gold["ties_d2"]
     gi, gd = handle.knn(q)
     assert (bits(gd) == bits(rd)).all()                        # distances: bit-exact at every rank
     tied_queries = 0

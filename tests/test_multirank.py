@@ -143,10 +143,10 @@ def test_sharded_update_matches_oracle(flb, po, frames, tmp_path, mode):
     exchange."""
     import torch
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs >= 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs >= 2 GPUs")
     import torch.multiprocessing as mp
     out = str(tmp_path / "gpu.npz")
-    # FLB_TEST_WORLD=4 / 8 on a box with that many GPUs (gpurun --gpus N): the same test at that world size
+    # FLB_TEST_WORLD=4 / 8 on a machine with that many GPUs: the same test at that world size
     world = max(2, min(int(os.environ.get("FLB_TEST_WORLD", "2")), torch.cuda.device_count(), 8))
     mp.spawn(_gpu_worker, args=(world, _free_port(), out, mode), nprocs=world, join=True)
     r = np.load(out)
