@@ -171,6 +171,7 @@ struct flb_handle {
     DevBuf<float> map_raw_alt;
     DevBuf<unsigned char> dead, ins;
     DevBuf<int> dead_before, merge_counts, bbox_dev;
+    DevBuf<int> vox_unclean, vox_rep, vox_counts;  // Add_Points voxels resolved by the one-thread replay (k_vox_replay*)
     float map_lo[3] = {0, 0, 0}, map_hi[3] = {0, 0, 0};   // tight bounding box of the live map points
     float grid_lo[3] = {0, 0, 0}, grid_hi[3] = {0, 0, 0}; // box the kNN grid covers (= map box + a margin for growth)
     // map maintenance scratch
@@ -936,6 +937,7 @@ int flb_destroy(flb_handle* h) {
     h->map_comb.release(); h->boxes.release(); h->vkeys.release(); h->vkeys_sorted.release(); h->keep.release(); h->sel_idx.release();
     h->map_pts_alt.release(); h->cell_start_alt.release(); h->map_raw_alt.release(); h->dead.release(); h->ins.release();
     h->dead_before.release(); h->merge_counts.release(); h->bbox_dev.release();
+    h->vox_unclean.release(); h->vox_rep.release(); h->vox_counts.release();
     h->cub_tmp.release(); h->map_pts.release(); h->cell_start.release(); h->scan.release(); h->sel.release();
     h->plane_ok.release(); h->plane.release(); h->x_world.release(); h->x_nn_d2.release(); h->x_pd2.release();
     h->x_nn_idx.release(); h->x_rowmask.release(); h->x_rows.release(); h->x_meas.release(); h->partials.release();
@@ -1136,6 +1138,10 @@ static int map_add_points_full(flb_handle* h, const float* st, int n, float down
     FLB_CUDA(h, h->vals.reserve(total));
     FLB_CUDA(h, h->vals_sorted.reserve(total));
     FLB_CUDA(h, h->keep.reserve(total));
+    FLB_CUDA(h, h->vox_unclean.reserve(total));
+    FLB_CUDA(h, h->vox_rep.reserve(total));
+    FLB_CUDA(h, h->vox_counts.reserve(2));
+    FLB_CUDA(h, cudaMemsetAsync(h->vox_counts.p, 0, 2 * sizeof(int), h->stream));
     FLB_CUDA(h, cudaMemcpyAsync(h->map_comb.p, h->map_raw.p, (size_t)M * 3 * sizeof(float), cudaMemcpyDeviceToDevice, h->stream));
     FLB_CUDA(h, cudaMemcpyAsync(h->map_comb.p + (size_t)M * 3, st, (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
     FLB_CUDA(h, h->st_map.mark(h->stream));
@@ -1154,9 +1160,14 @@ static int map_add_points_full(flb_handle* h, const float* st, int n, float down
     h->launches += 4;
     {
         LaunchScope ls(h, FAM_OTHER);
+        k_vox_unclean<<<nb, 256, 0, h->stream>>>(h->vals_sorted.p, h->map_comb.p, total, downsample_size, h->vox_unclean.p,
+                                                  h->vox_counts.p);
         k_vox_resolve<<<nb, 256, 0, h->stream>>>(h->vkeys_sorted.p, h->vals_sorted.p, h->map_comb.p, total, M, downsample_size,
-                                                  h->keep.p);
+                                                  h->vox_unclean.p, h->vox_counts.p, h->vox_rep.p, h->keep.p);
+        k_vox_replay<<<1, 1, 0, h->stream>>>(h->vkeys_sorted.p, h->vals_sorted.p, h->map_comb.p, total, downsample_size, h->vox_unclean.p,
+                                             h->vox_counts.p, h->vox_rep.p, h->keep.p);
         FLB_CUDA(h, cudaGetLastError());
+        h->launches += 2;
     }
     return compact_and_rebuild(h, h->vals_sorted.p, total);
 }
@@ -1242,15 +1253,20 @@ int flb_map_add_points(flb_handle* h, const float* world_xyz, int n, int stride,
     FLB_CUDA(h, h->map_pts_alt.reserve((size_t)M + n));
     FLB_CUDA(h, h->map_raw_alt.reserve(((size_t)M + n) * 3));
     FLB_CUDA(h, h->cell_start_alt.reserve((size_t)ncell + 1));
+    FLB_CUDA(h, h->vox_unclean.reserve(n));
+    FLB_CUDA(h, h->vox_rep.reserve(n));
+    FLB_CUDA(h, h->vox_counts.reserve(2));
     float* nxyz = h->map_comb.p;
     FLB_CUDA(h, cudaMemcpyAsync(nxyz, st, (size_t)n * 3 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
     FLB_CUDA(h, h->st_map.mark(h->stream));
     FLB_CUDA(h, cudaMemsetAsync(h->dead.p, 0, M, h->stream));
     FLB_CUDA(h, cudaMemsetAsync(h->ins.p, 0, n, h->stream));
+    FLB_CUDA(h, cudaMemsetAsync(h->vox_counts.p, 0, 2 * sizeof(int), h->stream));
     const int gn = (n + 255) / 256, gm = (M + 255) / 256;
     {
         LaunchScope ls(h, FAM_OTHER);
-        k_vox_keys_rel<<<gn, 256, 0, h->stream>>>(nxyz, n, ds, bx, by, bz, wx, wx + wy, h->vkeys.p, h->vals.p);
+        k_vox_keys_rel<<<gn, 256, 0, h->stream>>>(nxyz, n, ds, bx, by, bz, wx, wx + wy, h->vkeys.p, h->vals.p, h->vox_unclean.p,
+                                                   h->vox_counts.p);
         FLB_CUDA(h, cudaGetLastError());
     }
     size_t tmp_bytes = 0, t2 = 0, t3 = 0;
@@ -1265,7 +1281,10 @@ int flb_map_add_points(flb_handle* h, const float* world_xyz, int n, int stride,
     {
         LaunchScope ls(h, FAM_OTHER);
         k_vox_resolve_incremental<<<gn, 256, 0, h->stream>>>(h->vkeys_sorted.p, h->vals_sorted.p, nxyz, n, ds, g, h->cell_start.p, h->map_pts.p,
-                                                              h->dead.p, h->ins.p);
+                                                              h->vox_unclean.p, h->vox_counts.p, h->vox_rep.p, h->dead.p, h->ins.p);
+        k_vox_replay_incremental<<<1, 1, 0, h->stream>>>(nxyz, ds, g, h->cell_start.p, h->map_pts.p, h->vox_counts.p, h->vox_rep.p, h->dead.p,
+                                                         h->ins.p);
+        h->launches++;
         // inserted points sorted by grid cell (not-inserted ones sort behind every cell)
         k_insert_cells<<<gn, 256, 0, h->stream>>>(nxyz, n, h->ins.p, g, ncell, h->keys.p, h->vals.p);
         FLB_CUDA(h, cudaGetLastError());

@@ -239,7 +239,51 @@ __global__ void k_bbox(const float* __restrict__ xyz, int n, int* __restrict__ b
 // emptied and `result` put back.  Its net effect per voxel is order-independent up to ties, so the
 // device version sorts (existing + new) points by voxel and lets one thread replay that sequential
 // rule over each voxel's handful of points.
+//
+// That holds only while every point lies in exactly one float box.  The box of voxel k is
+// [fl(k*ds), fl(fl(k*ds) + ds)) per axis, so for a ds that is not a power of two neighbouring boxes can
+// overlap or leave a gap of an ulp: a point within a few ulps of a boundary can lie in two boxes, or in
+// none (not even its own).  Its fate then depends on the order in which the reference meets the points.
+// So a voxel is resolved in parallel only when it is "clean": every point involved lies in its own box
+// and in no neighbour's (vox_clean).  The other voxels ("dirty": a point lands within a few ulps of a
+// boundary about once in 10^4..10^5 per axis, so a real frame has none or a handful) are replayed by one
+// thread in submission order with the reference's sequential rule and its exact box test.
 // ---------------------------------------------------------------------------------------
+// p lies strictly in its own float box (ikd_Tree.cpp:392-397, half-open test of :998) and in no neighbour's
+__device__ __forceinline__ bool vox_clean(const float* p, float ds) {
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        const float kf = floorf(p[a] / ds);
+#pragma unroll
+        for (int d = -1; d <= 1; ++d) {
+            const float mn = __fmul_rn(kf + (float)d, ds), mx = __fadd_rn(mn, ds);
+            const bool in = mn <= p[a] && mx > p[a];
+            if (in != (d == 0)) return false;
+        }
+    }
+    return true;
+}
+__device__ __forceinline__ bool in_vox_box(const float* mn, const float* mx, float x, float y, float z) {
+    return mn[0] <= x && mx[0] > x && mn[1] <= y && mx[1] > y && mn[2] <= z && mx[2] > z;
+}
+// box and centre of the downsample voxel of p, float arithmetic as ikd_Tree.cpp:392-400 writes it
+__device__ __forceinline__ void vox_box(const float* p, float ds, float* mn, float* mx, float* mid) {
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        mn[a] = __fmul_rn(floorf(p[a] / ds), ds);
+        mx[a] = __fadd_rn(mn[a], ds);
+        mid[a] = (float)((double)mn[a] + (double)(mx[a] - mn[a]) / 2.0);
+    }
+}
+// the few dirty entries, sorted in place by `by[entry]` (submission order); one thread
+__device__ void sort_small_by(int* e, int n, const int* by) {
+    for (int i = 1; i < n; ++i) {
+        const int v = e[i];
+        int j = i - 1;
+        while (j >= 0 && (by ? by[e[j]] : e[j]) > (by ? by[v] : v)) { e[j + 1] = e[j]; --j; }
+        e[j + 1] = v;
+    }
+}
 __device__ __forceinline__ unsigned long long vox_key(float x, float y, float z, float ds) {
     // floor(p / downsample_size) per axis (ikd_Tree.cpp:392-396), biased into 21 bits each
     const long long ix = (long long)floorf(x / ds) + (1ll << 20), iy = (long long)floorf(y / ds) + (1ll << 20),
@@ -256,10 +300,20 @@ __global__ void k_vox_keys(const float* __restrict__ xyz, int total, float ds, u
     vals[i] = i;
 }
 
+// sorted positions of the points (existing and new) that are not clean; counts[0] must be zero on entry
+__global__ void k_vox_unclean(const int* __restrict__ vals, const float* __restrict__ xyz, int total, float ds,
+                              int* __restrict__ unclean, int* __restrict__ counts) {
+    const int j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= total) return;
+    if (!vox_clean(xyz + 3 * (size_t)vals[j], ds)) unclean[atomicAdd(counts, 1)] = j;
+}
+
 // keys/vals sorted by voxel (stable: ascending index inside a voxel, so existing points [idx < M] come
-// first and new points keep their submission order).  One thread per voxel segment.
+// first and new points keep their submission order).  One thread per voxel segment.  A dirty voxel keeps its
+// existing points, drops its new ones for now and queues them in rep[] for k_vox_replay (counts[1]).
 __global__ void k_vox_resolve(const unsigned long long* __restrict__ keys, const int* __restrict__ vals,
-                              const float* __restrict__ xyz, int total, int M, float ds, unsigned char* __restrict__ keep) {
+                              const float* __restrict__ xyz, int total, int M, float ds, const int* __restrict__ unclean,
+                              int* __restrict__ counts, int* __restrict__ rep, unsigned char* __restrict__ keep) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= total) return;
     const unsigned long long k = keys[i];
@@ -276,11 +330,21 @@ __global__ void k_vox_resolve(const unsigned long long* __restrict__ keys, const
     // box and centre from the first new point (ikd_Tree.cpp:392-400), float arithmetic as written there
     const int v0 = vals[first_new];
     float mn[3], mx[3], mid[3];
-#pragma unroll
-    for (int a = 0; a < 3; ++a) {
-        mn[a] = floorf(xyz[3 * (size_t)v0 + a] / ds) * ds;
-        mx[a] = mn[a] + ds;
-        mid[a] = (float)((double)mn[a] + (double)(mx[a] - mn[a]) / 2.0);
+    vox_box(xyz + 3 * (size_t)v0, ds, mn, mx, mid);
+    // dirty: a point of the voxel outside its box or inside a neighbour's, or a point of another voxel inside this box
+    bool dirty = false;
+    for (int j = i; j < end && !dirty; ++j) dirty = !vox_clean(xyz + 3 * (size_t)vals[j], ds);
+    const int nu = counts[0];
+    for (int u = 0; u < nu && !dirty; ++u) {
+        const float* p = xyz + 3 * (size_t)vals[unclean[u]];
+        dirty = in_vox_box(mn, mx, p[0], p[1], p[2]);
+    }
+    if (dirty) {
+        for (int j = i; j < end; ++j) {
+            keep[j] = vals[j] < M ? 1 : 0;
+            if (vals[j] >= M) rep[atomicAdd(counts + 1, 1)] = j;
+        }
+        return;
     }
     // content of the box: existing points that pass the half-open box test (:1001)
     int c = 0, best = -1;
@@ -315,6 +379,46 @@ __global__ void k_vox_resolve(const unsigned long long* __restrict__ keys, const
         for (int j = i; j < first_new; ++j)
             if (!keep[j]) keep[j] = 1;
         (void)best0;
+    }
+}
+
+// The new points of the dirty voxels, one at a time in submission order, with the reference's sequential rule
+// (ikd_Tree.cpp:390-418).  The live points of a dirty voxel's box are those of its own key segment that pass the box
+// test, plus unclean points of other voxels that do (a clean point lies in its own box only).  One thread.
+__global__ void k_vox_replay(const unsigned long long* __restrict__ keys, const int* __restrict__ vals, const float* __restrict__ xyz,
+                             int total, float ds, const int* __restrict__ unclean, int* __restrict__ counts, int* __restrict__ rep,
+                             unsigned char* __restrict__ keep) {
+    if (blockIdx.x != 0 || threadIdx.x != 0) return;
+    const int nr = counts[1], nu = counts[0];
+    if (nr == 0) return;
+    sort_small_by(rep, nr, vals);
+    for (int r = 0; r < nr; ++r) {
+        const int j = rep[r];
+        const float* p = xyz + 3 * (size_t)vals[j];
+        float mn[3], mx[3], mid[3];
+        vox_box(p, ds, mn, mx, mid);
+        const unsigned long long k = keys[j];
+        int s0 = j, s1 = j + 1;
+        while (s0 > 0 && keys[s0 - 1] == k) --s0;
+        while (s1 < total && keys[s1] == k) ++s1;
+        // two sweeps over Downsample_Storage: count + closest, then (if the box changes) delete all but the result
+        int c = 0, best = j;
+        float best_d = dist2f(p[0], p[1], p[2], mid[0], mid[1], mid[2]);
+        for (int pass = 0; pass < 2; ++pass) {
+            const bool del = pass == 1;
+            if (del && !(c > 1 || best == j)) break;                       // :412 false: nothing changes
+            for (int t = s0; t < s1 + nu; ++t) {
+                const int q = t < s1 ? t : unclean[t - s1];
+                if (!keep[q] || (t >= s1 && keys[q] == k)) continue;       // dead, or already seen in the segment
+                const float* o = xyz + 3 * (size_t)vals[q];
+                if (!in_vox_box(mn, mx, o[0], o[1], o[2])) continue;
+                if (del) { keep[q] = 0; continue; }
+                ++c;
+                const float d = dist2f(o[0], o[1], o[2], mid[0], mid[1], mid[2]);
+                if (d < best_d) { best_d = d; best = q; }
+            }
+            if (del) keep[best] = 1;
+        }
     }
 }
 
@@ -353,10 +457,13 @@ __device__ __forceinline__ int grid_axis_cell(float v, float o, float inv_cell, 
     const int c = (int)floorf((v - o) * inv_cell);
     return min(max(c, 0), n - 1);
 }
+// also lists the new points that are not clean (unclean[], counts[0]: zero on entry)
 __global__ void k_vox_keys_rel(const float* __restrict__ xyz, int n, float ds, int bx, int by, int bz, int sy, int sz,
-                               unsigned long long* __restrict__ keys, int* __restrict__ vals) {
+                               unsigned long long* __restrict__ keys, int* __restrict__ vals, int* __restrict__ unclean,
+                               int* __restrict__ counts) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
+    if (!vox_clean(xyz + 3 * (size_t)i, ds)) unclean[atomicAdd(counts, 1)] = i;
     // floor(p / ds) per axis (ikd_Tree.cpp:392-396) relative to the map box, packed x | y << sy | z << sz
     const long long ix = (long long)floorf(xyz[3 * (size_t)i] / ds) - bx, iy = (long long)floorf(xyz[3 * (size_t)i + 1] / ds) - by,
                     iz = (long long)floorf(xyz[3 * (size_t)i + 2] / ds) - bz;
@@ -365,8 +472,8 @@ __global__ void k_vox_keys_rel(const float* __restrict__ xyz, int n, float ds, i
 }
 __global__ void k_vox_resolve_incremental(const unsigned long long* __restrict__ keys, const int* __restrict__ vals,
                                           const float* __restrict__ nxyz, int n, float ds, GridDesc g, const int* __restrict__ cell_start,
-                                          const float4* __restrict__ pts, unsigned char* __restrict__ dead,
-                                          unsigned char* __restrict__ ins) {
+                                          const float4* __restrict__ pts, const int* __restrict__ unclean, int* __restrict__ counts,
+                                          int* __restrict__ rep, unsigned char* __restrict__ dead, unsigned char* __restrict__ ins) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     const unsigned long long k = keys[i];
@@ -375,11 +482,14 @@ __global__ void k_vox_resolve_incremental(const unsigned long long* __restrict__
     while (end < n && keys[end] == k) ++end;
     const int v0 = vals[i];
     float mn[3], mx[3], mid[3];
-#pragma unroll
-    for (int a = 0; a < 3; ++a) {
-        mn[a] = floorf(nxyz[3 * (size_t)v0 + a] / ds) * ds;
-        mx[a] = mn[a] + ds;
-        mid[a] = (float)((double)mn[a] + (double)(mx[a] - mn[a]) / 2.0);
+    vox_box(nxyz + 3 * (size_t)v0, ds, mn, mx, mid);
+    // dirty (see vox_clean): a new point of the voxel, or any point found in its box, is not clean
+    bool dirty = false;
+    for (int j = i; j < end && !dirty; ++j) dirty = !vox_clean(nxyz + 3 * (size_t)vals[j], ds);
+    const int nu = counts[0];
+    for (int u = 0; u < nu && !dirty; ++u) {
+        const float* p = nxyz + 3 * (size_t)unclean[u];
+        dirty = in_vox_box(mn, mx, p[0], p[1], p[2]);
     }
     // Downsample_Storage = live points in the half-open box (Search_by_range, :1001)
     const int cx0 = grid_axis_cell(mn[0], g.ox, g.inv_cell, g.nx), cx1 = grid_axis_cell(mx[0], g.ox, g.inv_cell, g.nx);
@@ -397,9 +507,15 @@ __global__ void k_vox_resolve_incremental(const unsigned long long* __restrict__
                     ++c;
                     const float d = dist2f(p.x, p.y, p.z, mid[0], mid[1], mid[2]);
                     if (d < best_d) { best_d = d; best = m; }
+                    const float o[3] = {p.x, p.y, p.z};
+                    dirty = dirty || !vox_clean(o, ds);
                 }
             }
         }
+    if (dirty) {                                    // leave the voxel to k_vox_replay_incremental
+        for (int j = i; j < end; ++j) rep[atomicAdd(counts + 1, 1)] = vals[j];
+        return;
+    }
     bool replaced = false;
     for (int j = i; j < end; ++j) {
         const float* p = nxyz + 3 * (size_t)vals[j];
@@ -422,6 +538,58 @@ __global__ void k_vox_resolve_incremental(const unsigned long long* __restrict__
             }
         }
     if (best <= -2) ins[vals[-(best + 2)]] = 1;
+}
+// The new points of the dirty voxels, one at a time in submission order, with the reference's sequential rule
+// (ikd_Tree.cpp:390-418): Downsample_Storage = live existing points of the box (through the grid) + new points the
+// replay has kept so far that lie in it (no clean voxel's point can: it lies in its own box only).  One thread.
+__global__ void k_vox_replay_incremental(const float* __restrict__ nxyz, float ds, GridDesc g, const int* __restrict__ cell_start,
+                                         const float4* __restrict__ pts, int* __restrict__ counts, int* __restrict__ rep,
+                                         unsigned char* __restrict__ dead, unsigned char* __restrict__ ins) {
+    if (blockIdx.x != 0 || threadIdx.x != 0) return;
+    const int nr = counts[1];
+    if (nr == 0) return;
+    sort_small_by(rep, nr, nullptr);
+    for (int r = 0; r < nr; ++r) {
+        const int v = rep[r];
+        const float* p = nxyz + 3 * (size_t)v;
+        float mn[3], mx[3], mid[3];
+        vox_box(p, ds, mn, mx, mid);
+        const int cx0 = grid_axis_cell(mn[0], g.ox, g.inv_cell, g.nx), cx1 = grid_axis_cell(mx[0], g.ox, g.inv_cell, g.nx);
+        const int cy0 = grid_axis_cell(mn[1], g.oy, g.inv_cell, g.ny), cy1 = grid_axis_cell(mx[1], g.oy, g.inv_cell, g.ny);
+        const int cz0 = grid_axis_cell(mn[2], g.oz, g.inv_cell, g.nz), cz1 = grid_axis_cell(mx[2], g.oz, g.inv_cell, g.nz);
+        int c = 0, best = -(v + 2);                 // >= 0: sorted position of an existing point; <= -2: -(index + 2) of a new one
+        float best_d = dist2f(p[0], p[1], p[2], mid[0], mid[1], mid[2]);
+        for (int pass = 0; pass < 2; ++pass) {
+            const bool del = pass == 1;
+            if (del && !(c > 1 || best == -(v + 2))) break;              // :412 false: nothing changes
+            for (int z = cz0; z <= cz1; ++z)
+                for (int y = cy0; y <= cy1; ++y) {
+                    const int row = (z * g.ny + y) * g.nx;
+                    const int s0 = cell_start[row + cx0], s1 = cell_start[row + cx1 + 1];
+                    for (int m = s0; m < s1; ++m) {
+                        const float4 q = pts[m];
+                        if (dead[m] || !in_vox_box(mn, mx, q.x, q.y, q.z)) continue;
+                        if (del) { dead[m] = 1; continue; }
+                        ++c;
+                        const float d = dist2f(q.x, q.y, q.z, mid[0], mid[1], mid[2]);
+                        if (d < best_d) { best_d = d; best = m; }
+                    }
+                }
+            for (int t = 0; t < r; ++t) {
+                const int u = rep[t];
+                const float* q = nxyz + 3 * (size_t)u;
+                if (!ins[u] || !in_vox_box(mn, mx, q[0], q[1], q[2])) continue;
+                if (del) { ins[u] = 0; continue; }
+                ++c;
+                const float d = dist2f(q[0], q[1], q[2], mid[0], mid[1], mid[2]);
+                if (d < best_d) { best_d = d; best = -(u + 2); }
+            }
+            if (del) {
+                if (best >= 0) dead[best] = 0;
+                else ins[-(best + 2)] = 1;
+            }
+        }
+    }
 }
 // cell id of every new point (ncell = "not inserted": sorts behind every real cell)
 __global__ void k_insert_cells(const float* __restrict__ nxyz, int n, const unsigned char* __restrict__ ins, GridDesc g, int ncell,

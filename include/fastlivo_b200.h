@@ -93,7 +93,11 @@ int flb_map_upload(flb_handle* h, const float* xyz, int M, int stride_floats);
  *   flb_map_add_points  == ikdtree.Add_Points(PointToAdd, true) with downsample_size = filter_size_map
  *                          (map_incremental, src/laserMapping.cpp:692-706; ikd_Tree.cpp:382-457): per
  *                          downsample voxel touched by a new point, only the point closest to the voxel
- *                          centre survives (existing or new); untouched voxels are left alone.
+ *                          centre survives (existing or new); untouched voxels are left alone.  Within a
+ *                          few ulps of a voxel boundary the float boxes the reference tests points against
+ *                          ([fl(k*ds), fl(fl(k*ds) + ds)) per axis) can overlap or leave a gap, and the
+ *                          result depends on the order of the new points: there the reference's rule is
+ *                          replayed point by point in submission order, with its exact box test.
  *   flb_map_delete_boxes == ikdtree.Delete_Point_Boxes(cub_needrm) (lasermap_fov_segment,
  *                          src/laserMapping.cpp:363-421; ikd_Tree.cpp:501-521): boxes nb x 6 floats
  *                          (min xyz, max xyz), half-open containment min <= p < max.
